@@ -7,6 +7,7 @@ One "step" = one DIR training step on one synthetic batch per GPU:
   -> Adam, all through this repo's public (reference-shaped) API.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B]   # our arm (N>1: under torchrun)
+  python bench.py ... --dump-outputs DIR                            # + what the last timed step computed, DIR/*.npy
   python bench.py --impl reference ...                              # the CPU arm (oracle port, host cores)
 
 Prints ONE JSON line (rank 0).
@@ -115,7 +116,7 @@ def _epoch_features(n=12208, seed=7):
 
 
 class _CpuArm:
-    """The reference's own modules (baseline/_ref, oracle/ref_step.py) when installed, else the port
+    """The reference's own modules (oracle/_ref, oracle/ref_step.py) when installed, else the port
     (oracle/train_ref.py); same step either way: ResNet-50 fwd (train-mode BN) -> FDS.smooth (epoch >= 2 tables) ->
     regressor -> LDS-weighted L1 -> backward -> Adam, fp32 on the host cores."""
 
@@ -128,7 +129,7 @@ class _CpuArm:
             self.kind = "reference"
             self.tr = ref_step.ReferenceTrainer(bucket_num=BUCKET_NUM, bucket_start=BUCKET_START, epoch_features=feats,
                                                 epoch_labels=lab)
-            self.what = "the reference's own resnet.py / fds.py / loss.py (baseline/_ref), torch fp32 CPU kernels"
+            self.what = "the reference's own resnet.py / fds.py / loss.py (oracle/_ref), torch fp32 CPU kernels"
         else:
             from oracle.train_ref import RefTrainer
             self.kind = "port"
@@ -137,7 +138,7 @@ class _CpuArm:
             tables = (torch.randn(nb, 2048, generator=g) * .1 + .5, torch.rand(nb, 2048, generator=g) + .5,
                       torch.randn(nb, 2048, generator=g) * .1 + .5, torch.rand(nb, 2048, generator=g) + .5)
             self.tr = RefTrainer(bucket_num=BUCKET_NUM, bucket_start=BUCKET_START, fds_tables=tables)
-            self.what = "oracle/train_ref.py (port: baseline/_ref not installed), torch fp32 CPU kernels"
+            self.what = "oracle/train_ref.py (port: oracle/_ref not installed), torch fp32 CPU kernels"
 
     def batch(self, bs):
         g = torch.Generator().manual_seed(0)
@@ -265,13 +266,32 @@ def make_batches(args, device, rank, ep_labels, w_all, pinned):
 
 def train_step(model, opt, x, t, w, epoch=2):
     from loss import weighted_l1_loss
-    outputs, _ = model(x, t, epoch)
+    outputs, encoding = model(x, t, epoch)
     loss = weighted_l1_loss(outputs, t, w)
     opt.zero_grad()
     loss.backward()
     model.reduce_gradients()
     opt.step()
-    return loss
+    return loss, outputs, encoding
+
+
+DUMP_SAMPLE = 1 << 22      # parameters / gradients written by --dump-outputs: 16 MB each as float32
+
+
+def dump_outputs(out_dir, loss, outputs, encoding, net):
+    """--dump-outputs: what one training step hands back -- the loss, the predictions, the encoding the forward
+    returns, the BatchNorm running statistics it updated, and the same fixed, seeded sample of the updated parameters
+    and of their gradients -- as float32 DIR/<name>.npy (~34 MB in all), so that two builds can be compared output for
+    output."""
+    os.makedirs(out_dir, exist_ok=True)
+    flat = net.flat_parameters()
+    idx = np.random.default_rng(0).choice(flat.numel(), size=min(DUMP_SAMPLE, flat.numel()), replace=False)
+    idx = torch.from_numpy(np.sort(idx)).to(flat.device)
+    running = [b.reshape(-1) for n, b in net.named_buffers() if ".running_" in n and not n.startswith("FDS.")]
+    arrays = {"loss": loss, "outputs": outputs, "encoding": encoding, "bn_running_stats": torch.cat(running),
+              "parameters_sample": flat[idx], "gradients_sample": net.flat_grads()[idx]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.detach().float().cpu().numpy())
 
 
 def timed(fn, steps, warmup, world, device):
@@ -427,9 +447,10 @@ def run_ours(args):
 
     # ---- (1) device-resident throughput: `value`
     dev_batches = make_batches(args, device, rank, ep_labels, w_all, pinned=False)
+    last = [None]
     def step_resident(i):
         x, t, w = dev_batches[i % len(dev_batches)]
-        train_step(model, opt, x, t, w)
+        last[0] = train_step(model, opt, x, t, w)
     sampler = ClockSampler(local)
     timed(step_resident, 0, args.warmup, world, device)
     launches0 = _lib.launch_count()
@@ -437,6 +458,9 @@ def run_ours(args):
     dev_ms, wall_ms = timed(step_resident, args.steps, 0, world, device)
     clocks = sampler.stop()
     launches = _lib.launch_count() - launches0
+    if args.dump_outputs and rank == 0:     # before the steps below change the model
+        dump_outputs(args.dump_outputs, *last[0], model.module)
+    last[0] = None
     ms_per_step = dev_ms / args.steps
     value = world * args.batch * args.steps / (dev_ms / 1e3)
 
@@ -458,7 +482,7 @@ def run_ours(args):
         (x, t, w), ev = slots[i % 2]
         torch.cuda.current_stream().wait_event(ev)
         prefetch(i + 1)
-        loss = train_step(model, opt, x, t, w)
+        loss = train_step(model, opt, x, t, w)[0]
         for a in (x, t, w):
             a.record_stream(torch.cuda.current_stream())
         if loss_events[i % 2] is not None:
@@ -559,7 +583,13 @@ def main():
     ap.add_argument("--cpu-batch", dest="cpu_batch", type=int, default=16,
                     help="images per step of the CPU arm (a bounded sample of the 256-image step)")
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps, write what the last of them computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

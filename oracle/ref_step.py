@@ -3,16 +3,17 @@ INFRASTRUCTURE ONLY (bench.py's `--impl reference` and `cpu_baseline` legs; noth
 this).
 
 The reference is pure Python (no build step, not pip-installable: no setup.py), so its "install" is a copy of the
-four files of the hot path -- agedb-dir/{resnet,fds,loss,utils}.py, identical to imdb-wiki-dir's -- made by
-__graft_entry__.build() into baseline/_ref/agedb-dir/ while /root/reference is visible (git-ignored, travels to the GPU
-box with the snapshot).  This module only adds the plumbing agedb-dir/train.py:246-262 has around them (train.py
+four files of the hot path -- agedb-dir/{resnet,fds,loss,utils}.py, identical to imdb-wiki-dir's -- into
+oracle/_ref/agedb-dir/ (git-ignored), made by __graft_entry__.build() when a checkout of the reference is readable at
+REFERENCE_ROOT (environment variable DIRB200_REFERENCE, else its default location); without one, build() goes on and
+the CPU arm runs the port.  This module only adds the plumbing agedb-dir/train.py:246-262 has around them (train.py
 itself cannot be imported: tensorboard_logger, argparse at import time):
 
     outputs, _ = model(inputs, targets, epoch); loss = weighted_l1_loss(outputs, targets, weights)
     optimizer.zero_grad(); loss.backward(); optimizer.step()
 
 on the host CPU in fp32.  `.cuda()` is shimmed to the identity (fds.py:52 calls it unconditionally; this arm must
-stay on the host cores even on a GPU box).  When baseline/_ref is absent, callers fall back to the port
+stay on the host cores even on a GPU box).  When oracle/_ref is absent, callers fall back to the port
 (oracle/train_ref.py) and say so (`kind: "port"`).
 """
 import importlib
@@ -23,7 +24,8 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DIR = os.path.join(ROOT, "baseline", "_ref", "agedb-dir")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref", "agedb-dir")
+REFERENCE_ROOT = os.environ.get("DIRB200_REFERENCE", "/root/reference")
 FILES = ("resnet.py", "fds.py", "loss.py", "utils.py")
 
 
@@ -31,8 +33,9 @@ def available():
     return all(os.path.exists(os.path.join(REF_DIR, f)) for f in FILES)
 
 
-def install(reference_root="/root/reference"):
-    """Copy the reference's hot-path modules into baseline/_ref (called by __graft_entry__.build())."""
+def install(reference_root=REFERENCE_ROOT):
+    """Copy the reference's hot-path modules into oracle/_ref (called by __graft_entry__.build()); False, and nothing
+    copied, when no checkout of the reference is readable at `reference_root`."""
     import shutil
     src = os.path.join(reference_root, "agedb-dir")
     if not os.path.isdir(src):
@@ -49,7 +52,7 @@ class ReferenceTrainer:
 
     def __init__(self, bucket_num=100, bucket_start=0, lr=1e-3, seed=0, epoch_features=None, epoch_labels=None):
         if not available():
-            raise RuntimeError("baseline/_ref is not populated (run __graft_entry__.build() where /root/reference exists)")
+            raise RuntimeError("oracle/_ref is not populated (run __graft_entry__.build() with the reference readable)")
         saved_path, saved_mods = list(sys.path), {k: sys.modules.get(k) for k in ("resnet", "fds", "loss", "utils")}
         saved_cuda = (torch.Tensor.cuda, torch.nn.Module.cuda)
         torch.Tensor.cuda = lambda self, *a, **k: self
@@ -104,4 +107,4 @@ class ReferenceTrainer:
             fds.smooth(xb, l[:256].reshape(-1, 1), 3)
             smo.append(time.perf_counter() - t0)
         return {"update_running_stats_ms": round(1e3 * sorted(upd)[1], 2), "smooth_b256_ms": round(1e3 * sorted(smo)[1], 2),
-                "rows": int(f.shape[0]), "impl": "reference fds.FDS (baseline/_ref)"}
+                "rows": int(f.shape[0]), "impl": "reference fds.FDS (oracle/_ref)"}

@@ -17,13 +17,20 @@ def test_reference_arm_prints_one_contract_line():
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["metric"] == "images/sec" and d["unit"] == "images/s"
     assert d["higher_is_better"] is True and d["value"] > 0 and d["steps"] == 1
-    # the reference's own modules when baseline/_ref is populated (build() does it wherever /root/reference exists)
-    have_ref = os.path.exists(os.path.join(ROOT, "baseline", "_ref", "agedb-dir", "fds.py"))
+    # the reference's own modules when oracle/_ref is populated (build() does it when the reference is readable)
+    have_ref = os.path.exists(os.path.join(ROOT, "oracle", "_ref", "agedb-dir", "fds.py"))
     assert d["cpu_baseline"]["kind"] == ("reference" if have_ref else "port") and d["cpu_baseline"]["cores"] >= 1
     assert "IMDB-WIKI" in d["config"]["workload"] and "fds_ms" in d["cpu_baseline"]
     assert d["cpu_baseline"]["value"] == d["value"] == d["e2e"]["value"]
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0
     assert "workload" in d["config"] and d["gpu_launches"] == 0
+
+
+def test_bench_rejects_zero_steps_and_a_dump_of_the_cpu_arm():
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True,
+                           timeout=600, cwd=ROOT)
+        assert r.returncode == 2 and extra[-2] in r.stderr, (extra, r.stderr[-2000:])
 
 
 def test_conv_flop_accounting_matches_survey():
